@@ -3,7 +3,7 @@
 iterativelength on an R-MAT scale-22 CSR (4M vertices / 64M edges, int32 on device), 1024 hashed
 src-dst pairs per GPU, with the edges-traversed roofline and the reference's CPU operator beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" = one pass of the hot path (pgq_iterativelength) over one batch of P pairs on the resident
@@ -12,6 +12,10 @@ stream, CUDA events); `e2e` starts from HOST columns with the copies inside the 
 the host-pointer C ABI (pgq_iterativelength: pairs H2D + results D2H inside the call), at N > 1
 sharding.ShardedLengths (pinned staging, H2D of all pairs, this rank's shard of the searches, one NCCL
 all_reduce(MAX) of the result column on the device, D2H).  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes, on rank 0, the result columns of the last timed step as DIR/<name>.npy: `length` (float64,
+-1 where there is no path) and `valid` (float32) of the headline, and `c3_*` / `c5_*` of the sub-records.  The
+graphs and pairs depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -119,6 +123,21 @@ def load_graph(scale: int, rank: int, world: int, dist):
     return datagen.rmat_edges_cached(scale, CACHE)
 
 
+DUMP_BYTES = 60 << 20  # the arrays of one dump; with the .npy headers well under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """arrays: name -> float32 / float64 array, written as out_dir/<name>.npy.  Above DUMP_BYTES in all, every
+    array keeps the same share of its rows, chosen by a fixed seed, so two runs still compare row for row."""
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, a.size * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # reference arm / cpu baseline: the reference's own CPU operator on this box's host cores
 # ------------------------------------------------------------------------------------------------
@@ -189,7 +208,12 @@ def main():
     ap.add_argument("--alpha", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the c3 / c5 sub-records (R-MAT-24 / R-MAT-26)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the result columns of the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU arm (--impl ours)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
 
@@ -320,6 +344,9 @@ def main():
     ms_total = float(ms.item())
     value = total_pairs * args.steps / (ms_total / 1e3)
     last_dev = d_len[(nsteps - 1) & 1].cpu().numpy()
+    # (at N > 1 d_val holds this rank's searches only; the assembled column says valid = length >= 0)
+    last_valid = d_val.cpu().numpy() if world == 1 else (last_dev >= 0).astype(np.uint8)
+    dumps = {"length": last_dev.astype(np.float64), "valid": last_valid.astype(np.float32)}
 
     # ---- e2e: host buffers through the C ABI (H2D pairs + D2H results inside), result assembly for N > 1
     sharded = sharding.ShardedLengths(csr, dev, pgq.Options(args.lanes, args.direction, args.alpha)) if world > 1 else None
@@ -367,7 +394,8 @@ def main():
         torch.cuda.empty_cache()
         for name, scale, pairs_total, lanes in (("c3", 24, 4096, 0), ("c5", 26, 512 * world, 512)):
             try:
-                extra[name] = run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, stream, args)
+                extra[name] = run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, stream, args,
+                                         dumps)
             except Exception as ex:  # a sub-record must never cost the headline line
                 extra[name] = {"error": f"{type(ex).__name__}: {ex}"[:300]}
 
@@ -448,16 +476,19 @@ def main():
                         "same_answer": best["reachable"] == info.get("reachable")}
             except Exception as ex:
                 line["e2e_query"] = {"error": f"{type(ex).__name__}: {ex}"[:300]}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
 
 
-def run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, stream, args):
+def run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, stream, args, dumps):
     """One of the north star's larger configurations on the same ranks: the graph is generated and built on
     every GPU (replicated CSR), the searches of ONE pair set are dealt over the ranks, all_reduce(MAX)
-    assembles the answer.  Timed like the headline: CUDA events, barrier on both sides, max over ranks."""
+    assembles the answer.  Timed like the headline: CUDA events, barrier on both sides, max over ranks, --steps
+    calls.  The result columns of the last call go to dumps[name + "_length" / "_valid"]."""
     import torch
     from duckpgq_extension_b200 import pgq
     t0 = time.perf_counter()
@@ -484,7 +515,7 @@ def run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, str
 
     for _ in range(2):
         step()
-    reps = 3
+    reps = args.steps
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
@@ -513,6 +544,9 @@ def run_config(name, scale, pairs_total, lanes, ctx, dev, rank, world, dist, str
            "roofline_frac_rank0": (W * 4.0 / 1e9) / (ems / 1e3) / peak if ems > 0 else None,
            "pull_frac_rank0": (st["pull_edges"] * 4.0 / 1e9) / (st["pull_ms"] / 1e3) / peak if st["pull_ms"] > 0 else None,
            "reachable": int((d_len >= 0).sum().item()), "setup_s": setup_s, "csr_device_bytes": csr.info()[2]}
+    last_len = d_len.cpu().numpy()
+    dumps[f"{name}_length"] = last_len.astype(np.float64)
+    dumps[f"{name}_valid"] = (d_val.cpu().numpy() if world == 1 else last_len >= 0).astype(np.float32)
     csr.free()
     del d_src, d_dst, d_len, d_val
     torch.cuda.empty_cache()

@@ -8,7 +8,9 @@ set -euo pipefail
 REF=${REF:-/root/reference}
 HERE="$(cd "$(dirname "$0")" && pwd)"
 OUT="$HERE/build"
-BUILD=${BUILD:-/tmp/duckpgq_b200_build}
+# DuckDB's CMakeLists copies compile_commands.json into <build dir>/../../.cache/clangd, so the build dir sits
+# two levels below a directory of this user's own (a build dir right under /tmp would aim that copy at /.cache).
+BUILD=${BUILD:-${TMPDIR:-/tmp}/duckpgq_b200-$(id -u)/build/release}
 JOBS=${JOBS:-$(nproc)}
 if [ ! -d "$REF/duckdb/src" ]; then
   echo "reference sources not present at $REF - cannot build the DuckDB shim here" >&2; exit 0

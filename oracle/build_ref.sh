@@ -12,7 +12,9 @@ set -euo pipefail
 REF=${REF:-/root/reference}
 HERE="$(cd "$(dirname "$0")" && pwd)"
 OUT="$HERE/_ref"
-BUILD=${BUILD:-/tmp/duckpgq_ref_build}
+# DuckDB's CMakeLists copies compile_commands.json into <build dir>/../../.cache/clangd, so the build dir sits
+# two levels below a directory of this user's own (a build dir right under /tmp would aim that copy at /.cache).
+BUILD=${BUILD:-${TMPDIR:-/tmp}/duckpgq_ref-$(id -u)/build/release}
 JOBS=${JOBS:-$(nproc)}
 
 if [ -x "$OUT/duckdb" ] && [ -x "$OUT/unittest" ] && [ -z "${FORCE:-}" ]; then

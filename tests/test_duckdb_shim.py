@@ -3,22 +3,27 @@
   (b) duckpgq_extension_b200/duckdb_ext/build/duckdb_b200   the same + the duckpgq_b200 override,
       whose iterativelength / shortestpath callbacks run on the GPU through the C ABI
 and must return identical rows (hop counts, NULLs, element_id / vertices / edges lists, error
-texts).  Both binaries are built in the build container (oracle/build_ref.sh,
-duckdb_ext/build.sh) and travel to the GPU box; the test is skipped where they are absent."""
+texts).  What (a) returned is stored in tests/golden/duckdb_reference.json.gz (make_golden_duckdb.py);
+(b) is built from the reference's sources by duckdb_ext/build.sh, and the tests skip where it is absent."""
+import gzip
+import json
 import os
 import subprocess
 
 import pytest
 
-from conftest import ROOT
+from conftest import GOLDEN, ROOT
 
 pytestmark = pytest.mark.gpu
 
-REF = os.path.join(ROOT, "oracle", "_ref", "duckdb")
 B200 = os.path.join(ROOT, "duckpgq_extension_b200", "duckdb_ext", "build", "duckdb_b200")
 
-needs_binaries = pytest.mark.skipif(not (os.path.exists(REF) and os.path.exists(B200)),
-                                    reason="reference / shim DuckDB binaries not built")
+needs_binaries = pytest.mark.skipif(not os.path.exists(B200), reason="shim DuckDB binary not built")
+
+
+def reference_output():
+    with gzip.open(os.path.join(GOLDEN, "duckdb_reference.json.gz"), "rt") as f:
+        return json.load(f)
 
 
 def run(binary, sql):
@@ -114,7 +119,8 @@ def _undirected_rows(text):
 @pytest.mark.parametrize("case", sorted(CASES))
 def test_same_rows_as_reference(case):
     sql = CASES[case]
-    expected, expected_err = run(REF, sql)
+    ref = reference_output()["cases"][case]
+    expected, expected_err = ref["stdout"], ref["stderr"]
     got, got_err = run(B200, sql + "\n.print ----PGQ_B200_STATS----\nSELECT duckpgq_b200_stats();")
     assert "----PGQ_B200_STATS----" in got, (got[-2000:], got_err[-2000:])
     body, stats = got.split("----PGQ_B200_STATS----\n")
@@ -134,15 +140,7 @@ def test_same_rows_as_reference(case):
         assert int(calls["csr_uploads"]) == 0 and int(calls["csr_device_builds"]) > 0 and int(calls["csr_chunks"]) > 0
 
 
-@needs_binaries
-def test_operator_time_through_duckdb():
-    """The drop-in at work on a graph of some size (262 144 vertices / 4.2 M hashed edges, 2048 pairs in
-    one DataChunk): same rows from both binaries; the time DuckDB's profiler attributes to the
-    Projection that evaluates iterativelength is recorded (gpurun_out/duckdb_operator_times.json).
-    A first, identical statement warms the process up (CUDA context creation and the lazy loading of the
-    kernels it uses cost about a second, once per process); the profiled one still pays the per-query CSR upload, exactly as a real session would."""
-    import json
-    setup = """
+OPERATOR_SQL = """
 SET threads TO 8;
 CREATE TABLE v AS SELECT i::BIGINT AS id FROM range(0, 262144) t(i);
 CREATE TABLE e AS SELECT (hash(i * 2 + 1) % 262144)::BIGINT AS src, (hash(i * 2 + 2) % 262144)::BIGINT AS dst FROM range(0, 4194304) t(i);
@@ -157,25 +155,34 @@ FROM p, (SELECT count(cte1.temp) * 0 AS temp FROM cte1) __x;
 PRAGMA disable_profiling;
 SELECT count(pgq_len), sum(pgq_len), sum(hash(i, pgq_len) % 1000003) FROM r;
 """
+
+
+def measure_operator_time(binary, prof):
+    """OPERATOR_SQL through `binary` -> (last output row, {iterativelength_projection_s, statement_s})."""
     from oracle import ref_runner as rr
-    times = {}
-    rows = {}
+    out, err = run(binary, OPERATOR_SQL.format(prof=prof))
+    assert "Error" not in err, err
+    bfs, total = rr._projection_seconds(open(prof).read())
+    return out.strip().splitlines()[-1], {"iterativelength_projection_s": bfs, "statement_s": total}
 
-    def measure(name, binary):
-        prof = f"/tmp/pgq_prof_{name}.json"
-        out, err = run(binary, setup.format(prof=prof))
-        assert "Error" not in err, err
-        rows[name] = out.strip().splitlines()[-1]
-        bfs, total = rr._projection_seconds(open(prof).read())
-        return {"iterativelength_projection_s": bfs, "statement_s": total}
 
-    times["reference"] = measure("reference", REF)
+@needs_binaries
+def test_operator_time_through_duckdb(tmp_path):
+    """The drop-in at work on a graph of some size (262 144 vertices / 4.2 M hashed edges, 2048 pairs in
+    one DataChunk): same rows from both binaries; the time DuckDB's profiler attributes to the
+    Projection that evaluates iterativelength is recorded (gpurun_out/duckdb_operator_times.json).
+    A first, identical statement warms the process up (CUDA context creation and the lazy loading of the
+    kernels it uses cost about a second, once per process); the profiled one still pays the per-query CSR upload, exactly as a real session would.
+    The reference's row and times are stored, with the host they were measured on."""
+    ref = reference_output()["operator_time"]
+    times = {"reference": {k: ref[k] for k in ("iterativelength_projection_s", "statement_s", "measured_on")}}
     # a fresh GPU box now and then stalls a process's first seconds on the device (seen once: 1.7 s for a
     # statement that takes 0.03 s in every other run): the best of up to three processes is the measurement
     attempts = []
     for _ in range(3):
-        attempts.append(measure("b200", B200))
-        assert rows["reference"] == rows["b200"]
+        row, t = measure_operator_time(B200, str(tmp_path / "profile.json"))
+        attempts.append(t)
+        assert row == ref["row"]
         if attempts[-1]["iterativelength_projection_s"] < times["reference"]["iterativelength_projection_s"]:
             break
     times["b200"] = min(attempts, key=lambda t: t["iterativelength_projection_s"])
