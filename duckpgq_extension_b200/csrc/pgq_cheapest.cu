@@ -8,6 +8,14 @@
 // atomicMin and re-sweeps only the vertices whose distances improved, to the same fixed point,
 // bit for bit.  "Unreachable" is the reference's own sentinel max/2 (l.15), added to like any other
 // number (no guard, as UpdateOneLane l.29-36 has none).
+//
+// The fixed point needs every edge checked once from every vertex's final distance.  A vertex is
+// re-swept after each improvement, so what remains is the first sweep: the reference relaxes every
+// vertex there, even one still at the sentinel.  With weights >= 0 such a vertex lowers nothing
+// (max/2 + w >= max/2 >= any distance), so only the sources start dirty.  With a negative weight
+// max/2 + w can be below max/2 -- a target no source reaches then has a cost, and with DOUBLE
+// weights (max/2 + -1e308) even a reached one can get cheaper -- so, when the CSR holds any weight
+// below zero (w_negative, set at finalize), every vertex starts dirty.
 #include <algorithm>
 #include <cstring>
 
@@ -77,17 +85,17 @@ __global__ void __launch_bounds__(256) k_bf_sweep(int64_t n, int L, const int32_
 			const u64 dk = *reinterpret_cast<volatile u64 *>(&dist[v * L + g + lane]);
 			for (int e = e0; e < e1; e++) {
 				const int u = adj[e];
-				u64 nk;
-				if (F64) {
-					nk = f64_key(key_f64(dk) + __longlong_as_double(w_bits[e]));
-				} else {
-					nk = (u64)((long long)dk + w_bits[e]);
-				}
 				u64 *slot = &dist[(int64_t)u * L + g + lane];
 				bool better;
 				if (F64) {
-					better = nk < *reinterpret_cast<volatile u64 *>(slot) && nk < atomicMin(slot, nk);
+					// "better" is decided on the doubles, as the reference's nw < dists[n]: false for a NaN sum,
+					// whose key (a NaN with the sign bit set, which the fp64 add passes through) sorts below
+					// every number's
+					const double c = key_f64(dk) + __longlong_as_double(w_bits[e]);
+					const u64 nk = f64_key(c);
+					better = c < key_f64(*reinterpret_cast<volatile u64 *>(slot)) && nk < atomicMin(slot, nk);
 				} else {
+					const u64 nk = (u64)((long long)dk + w_bits[e]);
 					better = (long long)nk < *reinterpret_cast<volatile long long *>(slot) &&
 					         (long long)nk < atomicMin(reinterpret_cast<long long *>(slot), (long long)nk);
 				}
@@ -164,7 +172,9 @@ static int run_bf(pgq_csr *csr, Workspace *ws, int64_t p, const int64_t *d_src, 
 		const int cnt = (int)std::min<int64_t>(L, p - b0);
 		k_bf_init<F64><<<(unsigned)std::min<int64_t>((dist_elems + 255) / 256, (int64_t)sms * 16), 256, 0, s>>>(
 		    (int64_t)dist_elems, dist);
-		PGQ_CUDA(cudaMemsetAsync(dirty, 0, dirty_bytes, s));
+		// with a negative weight every vertex is relaxed in the first sweep, sentinel or not (see the header);
+		// the bits past n in the last word are never read, the sweep stops at v < n
+		PGQ_CUDA(cudaMemsetAsync(dirty, csr->w_negative ? 0xff : 0, dirty_bytes, s));
 		k_bf_sources<F64><<<(cnt + 127) / 128, 128, 0, s>>>((int)b0, cnt, L, d_src, d_sv, csr->perm, n, dist, dirty,
 		                                                   flags + 1);
 		st->batches++;

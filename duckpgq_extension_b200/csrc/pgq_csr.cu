@@ -594,6 +594,16 @@ __global__ void k_gather_edges(const int32_t *__restrict__ perm, const int32_t *
 	}
 }
 
+// *flag = 1 if some weight is below zero (cheapest_path_length then relaxes every vertex, pgq_cheapest.cu)
+__global__ void k_any_negative(const int64_t *__restrict__ w_bits, int64_t count, bool f64, int *flag) {
+	for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x) {
+		const int64_t b = w_bits[i];
+		if (f64 ? __longlong_as_double(b) < 0.0 : b < 0) {
+			*flag = 1;
+		}
+	}
+}
+
 // offsets must be non-decreasing, start at 0 and end at m
 __global__ void k_check_offsets(const int32_t *__restrict__ off, int64_t n, int64_t m, int *err) {
 	for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i <= n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -1552,6 +1562,14 @@ static int finalize_from_rows(pgq_csr *csr, Workspace *ws, cudaStream_t s) {
 		k_gather_edges<<<grid_for(m, 256, 148 * 16), 256, 0, s>>>(perm_out, csr->st_dst, csr->st_eid, csr->st_w, m,
 		                                                       csr->out.adj, csr->edge_ids, csr->w_bits);
 		PGQ_CUDA(cudaGetLastError());
+		if (csr->w_bits) {
+			PGQ_CUDA(cudaMemsetAsync(d_err, 0, sizeof(int), s));
+			k_any_negative<<<grid_for(m, 256, 148 * 16), 256, 0, s>>>(csr->w_bits, m, csr->weight_type == 2, d_err);
+			PGQ_CUDA(cudaGetLastError());
+			int neg = 0;
+			PGQ_TRY(read_flag(d_err, s, &neg));
+			csr->w_negative = neg != 0;
+		}
 	}
 	PGQ_TRY(finish_csr(csr, ws, s));
 	PGQ_CUDA(cudaStreamSynchronize(s));

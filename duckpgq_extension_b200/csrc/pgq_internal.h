@@ -161,6 +161,7 @@ struct pgq_csr {
 	// edge weights in out-CSR position order (CSR::w / CSR::w_double, compressed_sparse_row.hpp:32-40)
 	int weight_type = 0; // 0 none, 1 BIGINT, 2 DOUBLE
 	int64_t *w_bits = nullptr;
+	bool w_negative = false; // some weight < 0 (-inf included; not -0.0 or a NaN), set at finalize
 	std::unordered_map<void *, size_t> allocs; // every device buffer of this CSR with its size (buffer cache)
 };
 

@@ -84,6 +84,7 @@ extern "C" int pgq_csr_clone(pgq_csr *csr, pgq_ctx *target, pgq_csr **out) {
 	c->staged = csr->staged;
 	c->edge_init = true;
 	c->weight_type = csr->weight_type;
+	c->w_negative = csr->w_negative;
 	Workspace *ws = nullptr;
 	int st = pgq_ws_acquire(target, &ws);
 	if (st != PGQ_OK) {

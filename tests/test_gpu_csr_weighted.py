@@ -43,10 +43,12 @@ def build_chunked(ctx, n, src, dst, eid, weight=None, chunk=2048):
 
 def per_vertex_sorted(v, e, w, n):
     """(edge, weight) pairs of every vertex in a canonical order: the order inside a vertex is the arrival order
-    of the rows at create_csr_edge, which for the reference binary is DuckDB's join output order."""
+    of the rows at create_csr_edge, which for the reference binary is DuckDB's join output order.  Weights as
+    bits (int64 view), so that NaNs compare and -0.0 differs from 0.0."""
     row = np.repeat(np.arange(n), np.diff(np.asarray(v[:n + 1], dtype=np.int64)))
-    order = np.lexsort((w, e, row))
-    return np.asarray(e)[order], np.asarray(w)[order]
+    wb = np.ascontiguousarray(w).view(np.int64)
+    order = np.lexsort((wb, e, row))
+    return np.asarray(e)[order], wb[order]
 
 
 @pytest.mark.parametrize("name", WEIGHTED)
@@ -64,12 +66,12 @@ def test_weighted_csr_and_cheapest_path_golden(gpu_ctx, name):
         assert np.array_equal(a, b)  # bit-exact, doubles too
     cost, valid, st = csr.cheapest_path_length(g["psrc"], g["pdst"])
     assert np.array_equal(valid, g["cost_valid"])
-    assert np.array_equal(cost[valid == 1], g["cost"][valid == 1])  # exact equality, also for DOUBLE sums
+    assert np.array_equal(cost[valid == 1].view(np.int64), g["cost"][valid == 1].view(np.int64))  # bits, also for DOUBLE sums
     # the restatement agrees with the reference binary as well (pins oracle/pgq_oracle.c's Bellman-Ford)
     v, e, ids, ow = orc.csr_build_weighted(n, src, dst, w)
-    assert np.array_equal(ow, got_w) and np.array_equal(e, de)  # device build == single-thread restatement, position by position
+    assert np.array_equal(ow.view(np.int64), got_w.view(np.int64)) and np.array_equal(e, de)  # device build == single-thread restatement, position by position, bits
     ocost, ovalid = orc.cheapest_path_length(n, v, e, ow, g["psrc"], g["pdst"])
-    assert np.array_equal(ovalid, g["cost_valid"]) and np.array_equal(ocost[ovalid == 1], g["cost"][ovalid == 1])
+    assert np.array_equal(ovalid, g["cost_valid"]) and np.array_equal(ocost[ovalid == 1].view(np.int64), g["cost"][ovalid == 1].view(np.int64))
     # iterativelength2 is served by the same searches as iterativelength
     out, ov, _ = csr.iterativelength(g["psrc"], g["pdst"])
     assert np.array_equal(ov, g["length2_valid"]) and np.array_equal(out, g["length2"])

@@ -142,10 +142,12 @@ WEIGHTED = sorted(f[5:-4] for f in os.listdir(GOLDEN) if f.startswith("refw_") a
 
 def per_vertex_sorted(v, e, w, n):
     """(edge, weight) pairs of every vertex in a canonical order: the order inside a vertex is the arrival order
-    of the rows at create_csr_edge, which for the reference binary is DuckDB's join output order."""
+    of the rows at create_csr_edge, which for the reference binary is DuckDB's join output order.  Weights as
+    bits (int64 view), so that NaNs compare and -0.0 differs from 0.0."""
     row = np.repeat(np.arange(n), np.diff(np.asarray(v[:n + 1], dtype=np.int64)))
-    order = np.lexsort((w, e, row))
-    return np.asarray(e)[order], np.asarray(w)[order]
+    wb = np.ascontiguousarray(w).view(np.int64)
+    order = np.lexsort((wb, e, row))
+    return np.asarray(e)[order], wb[order]
 
 
 @pytest.mark.parametrize("name", WEIGHTED)
@@ -160,7 +162,7 @@ def test_weighted_csr_cheapest_path_and_iterativelength2_golden(name):
     for a, b in zip(per_vertex_sorted(v, e, ow, n), per_vertex_sorted(z["csr_v"], z["csr_e"].astype(np.int64), z["csr_w"], n)):
         assert np.array_equal(a, b)  # weights bit-exact, doubles too
     cost, valid = orc.cheapest_path_length(n, v, e, ow, ps, pd)
-    assert np.array_equal(valid, z["cost_valid"]) and np.array_equal(cost[valid == 1], z["cost"][valid == 1])
+    assert np.array_equal(valid, z["cost_valid"]) and np.array_equal(cost[valid == 1].view(np.int64), z["cost"][valid == 1].view(np.int64))
     out, ov, _ = orc.iterativelength2(n, v, e, ps, pd)
     assert np.array_equal(ov, z["length2_valid"]) and np.array_equal(out, z["length2"].astype(np.int64))
     out1, ov1, _ = orc.iterativelength(n, v, e, ps, pd)  # the two formulations answer alike
